@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (libcrisper.so kernels)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own path: HF pipeline on the host CPU
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's outputs as DIR/<name>.npy
 
 Workload: one GPU = BASELINE.json configs[1] (batch = 8 x 30 s synthetic 16 kHz chunks); several GPUs = configs[3]'s share
 (32 chunks per GPU, round-robin, decode batches of 16, transcript all_gather inside the timed region).  CrisperWhisper-
@@ -124,6 +125,22 @@ def synth_wave(seed: int, n: int = 480000) -> np.ndarray:
     return (np.random.default_rng(seed).standard_normal(n) * 0.1).astype(np.float32)
 
 
+def write_outputs(out_dir: str, arrays: dict, limit: int = 64_000_000) -> None:
+    """Save each [chunks, ...] array as out_dir/<name>.npy in float32 (token ids and frame indices are exact there).
+    Past `limit` bytes in all, every array keeps the same seeded sample of chunks, whose indices go to chunk_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.cpu().numpy().astype(np.float32) for k, v in arrays.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(a[0].nbytes for a in host.values()) + 4
+    keep = min(n, (limit - 4096) // row_bytes)
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        host = {k: a[idx] for k, a in host.items()}
+        host["chunk_index"] = idx.astype(np.float32)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------------------
 def run_reference(args, rank, world):
     """The reference's own implementation of the path: HF transformers pipeline on the host CPU (REF/transcribe.py:8-34
@@ -202,7 +219,13 @@ def main():
     ap.add_argument("--ref-warmup", dest="ref_warmup", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the per-stage / per-config measurements")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's tokens and DTW jump indices of every chunk to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "crisper":
+        ap.error("--dump-outputs applies to --impl crisper")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -217,11 +240,7 @@ def main():
     torch.cuda.set_device(local_rank)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
-    import __graft_entry__ as ge
-    if rank == 0 or world == 1:
-        ge.build()
-    if world > 1:
-        dist.barrier()
+    # the library __graft_entry__.build() left in the tree; the bench never compiles, so the tree may be read-only
     from crisperwhisper_b200 import _lib as L
     from crisperwhisper_b200 import distributed as D
     from crisperwhisper_b200 import weights as Wt
@@ -309,10 +328,19 @@ def main():
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     ev0.record(eng.stream)
     for _ in range(args.steps):
-        run_chunks(wave_dev, Bd, T, gather=True)
+        outs = run_chunks(wave_dev, Bd, T, gather=True)
     ev1.record(eng.stream)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs:
+        dumped = {"tokens": torch.cat([o[0] for o in outs]), "jump_indices": torch.cat([o[1] for o in outs])}
+        if world > 1:   # every rank's chunks in global order: local chunk i of rank r is chunk i * world + r
+            for k, t in dumped.items():
+                parts = [torch.empty_like(t) for _ in range(world)]
+                dist.all_gather(parts, t)
+                dumped[k] = torch.stack(parts, 1).flatten(0, 1)
+        if rank == 0:
+            write_outputs(args.dump_outputs, dumped)
     gpu_launches = eng.launch_count() - launches0
     ms_per_step = max_over_ranks(ev0.elapsed_time(ev1) / args.steps)
     audio_s = 30.0 * NC * world
